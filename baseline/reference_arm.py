@@ -1,7 +1,7 @@
 """Reference arm of the headline benchmark (``bench.py --impl reference``).
 
-Runs the UNMODIFIED reference package installed at ``baseline/_ref`` (``pip install --no-deps
---target`` of /root/reference) through its own public API and stock code path:
+Runs the UNMODIFIED reference package that ``build()`` installs at ``oracle/_ref``
+(``oracle/build_reference.py``) through its own public API and stock code path:
 
 * one ``ArraysToArraysService(wrap_logp_grad_func(f))`` gRPC worker PROCESS per data shard
   (the reference's deployment model, ``/root/reference/demo_node.py:98-108``), placed on the
@@ -28,14 +28,14 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 METRIC = "logp+grad evals/sec for 8-shard federated GLM"
 NOTE = (
-    "unmodified reference code from baseline/_ref (pip --no-deps); its third-party deps betterproto/grpclib "
+    "unmodified reference code from oracle/_ref (oracle/build_reference.py); its third-party deps betterproto/grpclib "
     "have no offline wheel and are provided as API shims over grpcio (baseline/shims); worker compute is stock "
     "PyTorch (bf16 matmuls); timing is wall clock around the client's gather (this path has no single device stream)"
 )
 
 
 def _paths():
-    for p in (os.path.join(HERE, "_ref"), os.path.join(HERE, "shims")):
+    for p in (os.path.join(ROOT, "oracle", "_ref"), os.path.join(HERE, "shims")):
         if p not in sys.path:
             sys.path.insert(0, p)
 
@@ -100,7 +100,7 @@ def main(args) -> None:
         import pytensor_federated  # noqa: F401  (the reference)
         from pytensor_federated import LogpGradServiceClient
     except Exception as ex:  # noqa: BLE001
-        print(json.dumps({"impl": "reference", "unavailable": f"cannot import the reference from baseline/_ref: {ex}"}))
+        print(json.dumps({"impl": "reference", "unavailable": f"cannot import the reference from oracle/_ref: {ex}"}))
         return
     import numpy as np
     import torch
@@ -140,7 +140,7 @@ def main(args) -> None:
             return
         if rank == 0:
             sys.path.insert(0, ROOT)
-            from bench import ClockSampler  # only the nvidia-smi sampler, nothing of the product path
+            from bench import ClockSampler, dump_outputs  # the clock sampler and the .npy writer, nothing of the product path
 
             clients = [LogpGradServiceClient("127.0.0.1", base_port + s) for s in range(args.shards)]
             rng = np.random.default_rng(7)
@@ -165,10 +165,12 @@ def main(args) -> None:
             checksum = 0.0
             t0 = time.perf_counter()
             for i in range(args.steps):
-                logp, _, _ = loop.run_until_complete(evaluate(thetas[args.warmup + i]))
+                logp, d_ic, d_beta = loop.run_until_complete(evaluate(thetas[args.warmup + i]))
                 checksum += logp
             elapsed = time.perf_counter() - t0
             clocks = sampler.stop()
+            if getattr(args, "dump_outputs", None):
+                dump_outputs(args.dump_outputs, [np.asarray(logp), d_ic, d_beta])
             value = args.steps / elapsed
             line = {
                 "metric": METRIC,

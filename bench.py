@@ -2,7 +2,8 @@
 
 Config (BASELINE.json): 8 shards x 10M rows x 256 features, bf16 design matrix, one theta per
 evaluation; shards are spread over the N GPUs (8/N per GPU => strong scaling).  Synthetic data,
-random parameters.  Contract: see the driver's instructions (one JSON line on rank 0).
+random parameters.  Rank 0 prints one JSON line; ``--dump-outputs DIR`` also writes what the last timed step
+returned, one ``DIR/<name>.npy`` (float64) per array, so that two builds can be compared output for output.
 
     python bench.py                       # N=1, default steps
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 \
@@ -30,7 +31,9 @@ METRIC = "logp+grad evals/sec for 8-shard federated GLM"   # the headline; the o
 def parse_args():
     p = argparse.ArgumentParser()
     p.add_argument("--gpus", type=int, default=1)
-    p.add_argument("--steps", type=int, default=30)
+    p.add_argument("--steps", type=int, default=100,
+                   help="timed evaluations; the default keeps the N = 1 headline region near 0.5 s, long enough to run "
+                        "at the clocks the power cap sustains")
     p.add_argument("--warmup", type=int, default=5)
     p.add_argument("--impl", default="b200", choices=["b200", "reference", "nccl"])
     p.add_argument("--rows", type=int, default=10_000_000, help="rows per shard")
@@ -42,13 +45,13 @@ def parse_args():
                    help="BASELINE.json configuration (glm = the headline; --kernel fp8 is an alias of --config fp8)")
     p.add_argument("--series", type=int, default=20_000, help="ode: time series per shard")
     p.add_argument("--timepoints", type=int, default=32, help="ode: observations per series")
-    p.add_argument("--min-seconds", type=float, default=0.5,
-                   help="the S-step block is repeated until the timed region lasts this long; the median block counts")
     p.add_argument("--speculative-us", type=float, default=1000.0,
                    help="e2e region: FederatedEngine.set_speculative(wait_us) — the next evaluation's kernel is enqueued "
                         "before theta exists (0 = one launch per evaluation only)")
     p.add_argument("--nuts-draws", type=int, default=200, help="linreg: draws (= tune) of the NUTS run")
     p.add_argument("--out", default=None, help="also append the JSON line to this file")
+    p.add_argument("--dump-outputs", default=None, metavar="DIR",
+                   help="write the arrays the last timed step returned (logp, then one gradient per input) as DIR/<name>.npy")
     return p.parse_args()
 
 
@@ -327,49 +330,41 @@ def run_b200(args):
             print(json.dumps({"error": "verification failed", "max_rel_err": max_rel, "tolerance": tol, "n_gpus": world}),
                   flush=True)
         thetas = [draw_theta() for _ in range(W + S)]
-        # ---- warm-up through the public API, and a first estimate of the step time --------------------------
+        # ---- warm-up through the public API -------------------------------------------------------------------
         share(W)
-        t0 = time.perf_counter()
         for i in range(W):
             eng.evaluate(*thetas[i])
-        est = max((time.perf_counter() - t0) / max(W, 1), 1e-6)
         barrier()
-        # the timed regions last at least --min-seconds: the S-step block is repeated, the MEDIAN block is reported
-        blocks = max(1, int(np.ceil(args.min_seconds / (est * S)))) if args.min_seconds > 0 else 1
-        blocks = min(blocks, 2000)
-        share(blocks * S)
+        share(S)
         sampler = ClockSampler(local_rank).start()
-        # ---- device-timed region: `blocks` x S back-to-back fused evaluations --------------------------------
-        block_ms = []
+        # ---- device-timed region: S back-to-back fused evaluations ---------------------------------------------
+        start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         if backend == "fused":
             stream = eng.torch_stream()
             eng.set_device_theta(thetas[W], enable=True)
             launches0 = eng.kernel_launches
-            events = [torch.cuda.Event(enable_timing=True) for _ in range(blocks + 1)]
-            events[0].record(stream)
+            start.record(stream)
             last = 0
-            for bi in range(blocks):
-                for _ in range(S):
-                    last = eng.launch()
-                events[bi + 1].record(stream)
-            eng.wait(last)
-            events[-1].synchronize()
-            block_ms = [events[i].elapsed_time(events[i + 1]) for i in range(blocks)]
-            launches = (eng.kernel_launches - launches0) // blocks
+            for _ in range(S):
+                last = eng.launch()
+            end.record(stream)
+            last_vals, last_theta = np.array(eng.wait(last), dtype=np.float64), thetas[W]
+            end.synchronize()
+            launches = eng.kernel_launches - launches0
             eng.set_device_theta(thetas[W], enable=False)
         else:
-            events = [torch.cuda.Event(enable_timing=True) for _ in range(blocks + 1)]
-            events[0].record()
-            for bi in range(blocks):
-                for i in range(S):
-                    eng.evaluate_raw(thetas[W + i])
-                events[bi + 1].record()
-            events[-1].synchronize()
-            block_ms = [events[i].elapsed_time(events[i + 1]) for i in range(blocks)]
+            start.record()
+            for i in range(S):
+                last_vals, last_theta = eng.evaluate_raw(thetas[W + i]), thetas[W + i]
+            end.record()
+            end.synchronize()
             launches = 0
+        timed_ms = start.elapsed_time(end)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, model.unpack_result(last_vals, model.call_context(last_theta)))
         barrier()
         # ---- end-to-end region: public API, pinned H2D of theta + D2H of the result each step -----------------
-        e2e_steps = share(blocks * S)
+        e2e_steps = share(S)
 
         evaluated = [0]   # evaluations of the current phase (the peers serve exactly as many as the root announced)
 
@@ -422,8 +417,8 @@ def run_b200(args):
             else:
                 spec_on = False
         clocks = sampler.stop()
-        result = dict(block_ms=block_ms, e2e_s=e2e_s, e2e_steps=e2e_steps, launches=launches, checksum=checksum,
-                      clocks=clocks, verified=verified, max_rel_err=max_rel, blocks=blocks, e2e_plain_s=e2e_plain_s,
+        result = dict(timed_ms=timed_ms, e2e_s=e2e_s, e2e_steps=e2e_steps, launches=launches, checksum=checksum,
+                      clocks=clocks, verified=verified, max_rel_err=max_rel, e2e_plain_s=e2e_plain_s,
                       e2e_speculative=spec_on, e2e_spec_s=locals().get("e2e_spec_s"))
     else:
         # peers: each phase serves exactly as many epochs as the root evaluates; their kernels wait on the
@@ -462,9 +457,7 @@ def run_b200(args):
     if rank != 0:
         return
 
-    block_ms = sorted(result["block_ms"])
-    med_ms = block_ms[len(block_ms) // 2]
-    ms_per_step = med_ms / S
+    ms_per_step = result["timed_ms"] / S
     value = 1000.0 / ms_per_step * K
     e2e_value = result["e2e_steps"] / result["e2e_s"] * K
     peaks = {}
@@ -483,9 +476,7 @@ def run_b200(args):
         "kernel": args.kernel if args.config == "glm" else args.config,
         "backend": backend,
         "comm": comm_mode,
-        "timed_blocks": result["blocks"],
-        "timed_seconds": sum(result["block_ms"]) / 1e3,
-        "block_ms_min_med_max": [block_ms[0], med_ms, block_ms[-1]],
+        "timed_seconds": result["timed_ms"] / 1e3,
         "hbm_bytes_per_eval_per_gpu": bytes_per_eval,
     }
     if bytes_per_eval:
@@ -542,6 +533,16 @@ def run_b200(args):
     if not result["verified"]:
         raise SystemExit(3)
     return line
+
+
+def dump_outputs(out_dir, arrays):
+    """``logp.npy``, ``grad_0.npy``, ... (float64): what a caller of the evaluation receives."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    names = ["logp"] + [f"grad_{i}" for i in range(len(arrays) - 1)]
+    for name, a in zip(names, arrays):
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(a, dtype=np.float64))
 
 
 def linreg_nuts(eng, args):

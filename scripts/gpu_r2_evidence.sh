@@ -18,9 +18,9 @@ timeout 600 python benchmarks/bench_batching_gpu.py --chains 8 16 --evals 300 --
 timeout 600 python benchmarks/bench_configs.py --out $OUT/configs_misc_r2.jsonl > $OUT/bench_configs_ev.log 2>&1; tail -3 $OUT/bench_configs_ev.log | cut -c1-300
 # every launch with its device time, then one full capture per tensor-core kernel
 timeout 600 ncu --metrics gpu__time_duration.sum --clock-control none -k regex:fed_ -c 40 --csv --log-file $OUT/launches_r2.csv \
-    python bench.py --shards 2 --steps 3 --warmup 3 --min-seconds 0 > $OUT/ncu_launches_r2.log 2>&1
+    python bench.py --shards 2 --steps 3 --warmup 3 > $OUT/ncu_launches_r2.log 2>&1
 timeout 900 ncu --set full --clock-control none --import-source on -k regex:fed_glm_tc -s 4 -c 1 -f -o $OUT/prof_tc_r2_final \
-    python bench.py --shards 2 --steps 2 --warmup 3 --min-seconds 0 > $OUT/ncu_tc_r2.log 2>&1; tail -2 $OUT/ncu_tc_r2.log
+    python bench.py --shards 2 --steps 2 --warmup 3 > $OUT/ncu_tc_r2.log 2>&1; tail -2 $OUT/ncu_tc_r2.log
 timeout 900 ncu --set full --clock-control none --import-source on -k regex:fed_glm_fp8 -s 4 -c 1 -f -o $OUT/prof_fp8_r2_final \
-    python bench.py --config fp8 --shards 2 --steps 2 --warmup 3 --min-seconds 0 > $OUT/ncu_fp8_r2.log 2>&1; tail -2 $OUT/ncu_fp8_r2.log
+    python bench.py --config fp8 --shards 2 --steps 2 --warmup 3 > $OUT/ncu_fp8_r2.log 2>&1; tail -2 $OUT/ncu_fp8_r2.log
 ls -la $OUT/*.ncu-rep
