@@ -42,12 +42,14 @@ constexpr int kRing = 16;            // published chunks the consumers may lag b
 constexpr int kLLRows = 16;          // epilogue warps at most (per-warp log-likelihood slots)
 
 struct SmemLayout {
-    uint32_t stages, stage_bytes, off_theta_b, theta_b_bytes, off_r, r_bytes, off_theta_f, off_icpt, off_ring,
+    uint32_t stages, stage_bytes, off_theta_b, theta_b_bytes, off_r, r_bytes, off_theta_f, off_icpt, off_phi, off_ring,
         off_bars, off_tmem, total, preload;
 };
 // r_bufs: residual (R) buffers between the epilogue and MMA #2 — 2 normally; 1 for 16 chains, where the 8 KB
-// buy the third TMA stage (the epilogue of 16 chains is long enough to hide the short MMA #2 it then waits for)
-__host__ __device__ inline SmemLayout smem_layout(int P, int n1, int n2, int n_theta, int n_groups, int chains, int r_bufs) {
+// buy the third TMA stage (the epilogue of 16 chains is long enough to hide the short MMA #2 it then waits for).
+// phi_bytes: the per-chain PhiChain table of the families with fitted parameters (0 otherwise).
+__host__ __device__ inline SmemLayout smem_layout(int P, int n1, int n2, int n_theta, int n_groups, int chains, int r_bufs,
+                                                 int phi_bytes = 0) {
     SmemLayout L;
     const uint32_t panels = P / kPanel;
     L.stage_bytes = panels * kPanelBytes;
@@ -55,8 +57,8 @@ __host__ __device__ inline SmemLayout smem_layout(int P, int n1, int n2, int n_t
     L.r_bytes = kTileM * n2 * 2;
     // theta (fp32) is staged inside the TMA stage ring and is dead once the bf16 B operand and the intercept
     // table are built, so it costs no shared memory of its own.
-    const uint32_t fixed = L.theta_b_bytes + r_bufs * L.r_bytes + ((chains * n_groups * 4 + 15) & ~15) + kRing * 24 + 192 +
-                           64 + 1024 /*alignment slack*/;
+    const uint32_t fixed = L.theta_b_bytes + r_bufs * L.r_bytes + ((chains * n_groups * 4 + 15) & ~15) + ((phi_bytes + 15) & ~15) +
+                           kRing * 24 + 192 + 64 + 1024 /*alignment slack*/;
     uint32_t stages = (227u * 1024u - fixed) / L.stage_bytes;
     if (stages > 4) stages = 4;
     L.stages = stages;
@@ -70,6 +72,7 @@ __host__ __device__ inline SmemLayout smem_layout(int P, int n1, int n2, int n_t
     L.off_theta_f = theta_in_last ? (stages - 1) * L.stage_bytes : 0;
     L.preload = theta_in_last ? stages - 1 : 0;
     L.off_icpt = o; o += (chains * n_groups * 4 + 15) & ~15;
+    L.off_phi = o; o += (phi_bytes + 15) & ~15;
     L.off_ring = o; o += kRing * 24;   // published chunks + one mbarrier per ring slot
     L.off_bars = o; o += 192;
     L.off_tmem = o; o += 64;
@@ -96,10 +99,10 @@ struct Cfg {
 };
 
 // doubles per CTA row of the partial array: (hi, lo) pairs of the n_vals outputs, then the per-warp slots of
-// the values that a whole warp contributes to — [kLLRows][n_out][KC][1 + G]: log-likelihood and the G
-// intercept gradients of every (output block, chain)
-__host__ __device__ constexpr size_t partial_row_doubles(int n_vals, int kc, int n_out, int n_groups) {
-    return 2 * ((size_t)n_vals + (size_t)kLLRows * n_out * kc * (1 + n_groups));
+// the values that a whole warp contributes to — [kLLRows][n_out][KC][1 + G + D]: log-likelihood, the G
+// intercept gradients and the D family-parameter gradients of every (output block, chain)
+__host__ __device__ constexpr size_t partial_row_doubles(int n_vals, int kc, int n_out, int n_groups, int n_family_params = 0) {
+    return 2 * ((size_t)n_vals + (size_t)kLLRows * n_out * kc * (1 + n_groups + n_family_params));
 }
 
 // (hi, lo) += x on a pair that only this thread touches during the launch
@@ -116,7 +119,11 @@ __device__ __forceinline__ void dd_accumulate(double* slot, double x) {
 // a statically assigned straggler.  Everything a chunk contributes (fp32 TMEM accumulation over its tiles,
 // per-thread fp32 sums) depends on the chunk alone, and chunk results are combined as double-double pairs
 // (fed::dd_add), so the evaluation stays reproducible although the assignment is not.
-template <int KC>
+//
+// kPhi: the families with fitted parameters (normal, student_t, negative_binomial; tc_common.cuh), selected at
+// run time among themselves.  theta = [intercept[G], beta[P], phi[D]] and the result [LL, gi[G], g[P], dphi[D]] per
+// chain; the D gradients fold exactly like LL.  A separate instantiation, so the other families keep their code.
+template <int KC, bool kPhi>
 __global__ void __launch_bounds__(Cfg<KC>::kThreads, 1)
 fed_glm_tc_kernel(FedComm comm, const GlmSegment* __restrict__ segs_g, GlmParams prm, const CUtensorMap* __restrict__ tmaps,
                   const GlmChunk* __restrict__ chunks, int n_chunks, unsigned int* __restrict__ work_counter) {
@@ -140,15 +147,18 @@ fed_glm_tc_kernel(FedComm comm, const GlmSegment* __restrict__ segs_g, GlmParams
     const int G = prm.n_groups;
     const int NH = PP / 128;          // 128-feature halves (UMMA M of MMA #2)
     const int panels = PP / kPanel;
-    const SmemLayout L = smem_layout(PP, N1, N2, comm.n_theta, G, KC, RB);
+    const SmemLayout L = smem_layout(PP, N1, N2, comm.n_theta, G, KC, RB, kPhi ? KC * (int)sizeof(PhiChain) : 0);
     const int S = (int)L.stages;
     const int nch = prm.n_chains < KC ? prm.n_chains : KC;  // chains actually present in theta
-    const int NV1 = 1 + G + P;        // outputs per chain: [LL, gi[G], g[P]]
+    const int D = kPhi ? prm.n_family_params : 0;
+    const int TS = G + P + D;         // theta per chain: [intercept[G], beta[P], phi[D]]
+    const int NV1 = 1 + G + P + D;    // outputs per chain: [LL, gi[G], g[P], dphi[D]]
 
     unsigned char* theta_b = smem + L.off_theta_b;
     unsigned char* r_buf = smem + L.off_r;
     float* theta_f = reinterpret_cast<float*>(smem + L.off_theta_f);  // valid until the setup barrier only
     float* icpt = reinterpret_cast<float*>(smem + L.off_icpt);        // [KC][G] intercepts
+    PhiChain* phi_tab = reinterpret_cast<PhiChain*>(smem + L.off_phi); // [KC] (kPhi only)
     int4* ring = reinterpret_cast<int4*>(smem + L.off_ring);          // (segment or -1, first row, tiles, -)
     uint64_t* bar_ring = reinterpret_cast<uint64_t*>(smem + L.off_ring + kRing * 16);   // slot j % kRing: chunk j published
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem + L.off_bars);
@@ -220,16 +230,20 @@ fed_glm_tc_kernel(FedComm comm, const GlmSegment* __restrict__ segs_g, GlmParams
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
     const int NOUT = prm.n_out;       // output blocks (1 = everything summed; else one per node)
-    const int NS1 = 1 + G;            // warp-level values per (block, chain): LL and the G intercept gradients
-    const size_t row_doubles = partial_row_doubles(comm.n_vals, KC, NOUT, G);
+    const int NS1 = 1 + G + D;        // warp-level values per (block, chain): LL, the G intercept and D phi gradients
+    const size_t row_doubles = partial_row_doubles(comm.n_vals, KC, NOUT, G, D);
     double* out = comm.cta_partials + (size_t)blockIdx.x * row_doubles;   // this CTA's running sums, (hi, lo) pairs
-    double* ll_slots = out + 2 * (size_t)comm.n_vals;                     // [kLLRows][NOUT][KC][1 + G] pairs
+    double* ll_slots = out + 2 * (size_t)comm.n_vals;                     // [kLLRows][NOUT][KC][1 + G + D] pairs
 
     if (active) {
         // ---------------- theta-dependent setup --------------------------------------------------
         for (size_t i = threadIdx.x; i < row_doubles / 2; i += blockDim.x) reinterpret_cast<double2*>(out)[i] = make_double2(0.0, 0.0);
         for (int i = threadIdx.x; i < KC * G; i += blockDim.x)
-            icpt[i] = (i / G) < nch ? theta_f[(i / G) * (G + P) + (i % G)] : 0.f;
+            icpt[i] = (i / G) < nch ? theta_f[(i / G) * TS + (i % G)] : 0.f;
+        if constexpr (kPhi) {
+            for (int k = threadIdx.x; k < KC; k += blockDim.x)
+                phi_tab[k] = k < nch ? phi_chain(prm.family, theta_f + k * TS + G + P) : PhiChain{0.0, 0.0, 0.0, {1.f, 1.f, 1.f, 1.f}};
+        }
         // Theta^T as the K-major, 128B-swizzled B operand of MMA #1: row n = 3*chain + term
         for (int idx = threadIdx.x; idx < panels * N1 * 8; idx += blockDim.x) {
             const int j = idx & 7;              // 16-byte chunk (8 features) within the 128-byte row
@@ -241,7 +255,7 @@ fed_glm_tc_kernel(FedComm comm, const GlmSegment* __restrict__ segs_g, GlmParams
 #pragma unroll
                 for (int e = 0; e < 8; ++e) {
                     const int f = pnl * kPanel + j * 8 + e;
-                    const float v = f < P ? theta_f[chain * (G + P) + G + f] : 0.f;
+                    const float v = f < P ? theta_f[chain * TS + G + f] : 0.f;
                     const __nv_bfloat16 hi = __float2bfloat16_rn(v);
                     const float rem1 = v - __bfloat162float(hi);
                     const __nv_bfloat16 mid = __float2bfloat16_rn(rem1);
@@ -428,8 +442,13 @@ fed_glm_tc_kernel(FedComm comm, const GlmSegment* __restrict__ segs_g, GlmParams
                     }
                 }
                 float ll_acc[KH], gi_cur[KH];
+                float ph_acc[kPhi ? KH : 1][2];   // row parts of dLL/dphi (kPhi)
 #pragma unroll
                 for (int k = 0; k < KH; ++k) ll_acc[k] = gi_cur[k] = 0.f;
+                if constexpr (kPhi) {
+#pragma unroll
+                    for (int k = 0; k < KH; ++k) ph_acc[k][0] = ph_acc[k][1] = 0.f;
+                }
                 for (int t = tp; t < ch.z; t += 2) {
                     const long long grow = (long long)ch.y + (long long)t * kTileM + row;
                     const bool valid = grow < seg_rows;
@@ -448,8 +467,16 @@ fed_glm_tc_kernel(FedComm comm, const GlmSegment* __restrict__ segs_g, GlmParams
                     for (int k = 0; k < KH; ++k) {
                         const float eta = (ev[3 * k] + ev[3 * k + 1]) + ev[3 * k + 2];
                         float ll = 0.f, r = 0.f;
-                        if (valid && (k0 + k) < nch)
-                            link_loglik(prm.family, y, eta + icpt[(k0 + k) * G + seg_group], ll, r);
+                        if constexpr (kPhi) {
+                            float d0 = 0.f, d1 = 0.f;
+                            if (valid && (k0 + k) < nch)
+                                link_loglik_phi(prm.family, y, eta + icpt[(k0 + k) * G + seg_group], phi_tab[k0 + k].p, ll, r, d0, d1);
+                            ph_acc[k][0] += d0;
+                            ph_acc[k][1] += d1;
+                        } else {
+                            if (valid && (k0 + k) < nch)
+                                link_loglik(prm.family, y, eta + icpt[(k0 + k) * G + seg_group], ll, r);
+                        }
                         ll_acc[k] += ll;
                         gi_cur[k] += r;
                         const __nv_bfloat16 hi = __float2bfloat16_rn(r);
@@ -526,6 +553,34 @@ fed_glm_tc_kernel(FedComm comm, const GlmSegment* __restrict__ segs_g, GlmParams
                             }
                     }
                 }
+                if constexpr (kPhi) {
+                    // dphi: the same fixed butterfly and the same per-warp slots (+ 1 + G + j).  The per-chain
+                    // constants of LL and dphi enter once per chunk, as (valid rows of the chunk) x c in fp64, from
+                    // the first warp of the chunk's even-tile group of these chains.
+                    const bool const_warp = tp == 0 && (ew & 3) == 0;
+                    const long long left = seg_rows - (long long)ch.y, span = (long long)ch.z * kTileM;
+                    const double n_valid = (double)(left < 0 ? 0 : (left < span ? left : span));
+#pragma unroll
+                    for (int k = 0; k < KH; ++k) {
+                        double s0 = (double)ph_acc[k][0], s1 = (double)ph_acc[k][1];
+#pragma unroll
+                        for (int o = 16; o > 0; o >>= 1) {
+                            s0 += __shfl_xor_sync(0xffffffffu, s0, o);
+                            s1 += __shfl_xor_sync(0xffffffffu, s1, o);
+                        }
+                        if (lane == 0 && (k0 + k) < nch) {
+                            double* slot = slot0 + 2 * (size_t)k * NS1;
+                            const PhiChain& pc = phi_tab[k0 + k];
+                            dd_accumulate(slot + 2 * (1 + G), s0);
+                            if (D > 1) dd_accumulate(slot + 2 * (2 + G), s1);
+                            if (const_warp) {
+                                dd_accumulate(slot, n_valid * pc.c_ll);
+                                dd_accumulate(slot + 2 * (1 + G), n_valid * pc.c_d0);
+                                if (D > 1) dd_accumulate(slot + 2 * (2 + G), n_valid * pc.c_d1);
+                            }
+                        }
+                    }
+                }
                 // gradient: the group that handled the chunk's last tile (odd index) drains the TMEM accumulator
                 if (tp == 1) {
                     const int gb = gbuf.idx;
@@ -567,8 +622,8 @@ fed_glm_tc_kernel(FedComm comm, const GlmSegment* __restrict__ segs_g, GlmParams
         tc_fence_after();
         fed::pdl_trigger();   // the next evaluation's CTA may take this SM as soon as we exit
         if (threadIdx.x == 0) fed::stamp(comm, 5);
-        // layout per (output block, chain): [LL, gi[G], g[P]] as (hi, lo) pairs; g[] was accumulated in place,
-        // LL and gi[] are the per-warp slots summed in warp order
+        // layout per (output block, chain): [LL, gi[G], g[P], dphi[D]] as (hi, lo) pairs; g[] was accumulated in
+        // place, LL, gi[] and dphi[] are the per-warp slots summed in warp order (slot 1 + G + j -> output 1 + G + P + j)
         for (int i = threadIdx.x; i < NOUT * nch * NS1; i += blockDim.x) {
             const int j = i % NS1, k = (i / NS1) % nch, o = i / (NS1 * nch);
             double hi = 0.0, lo = 0.0;
@@ -576,8 +631,9 @@ fed_glm_tc_kernel(FedComm comm, const GlmSegment* __restrict__ segs_g, GlmParams
                 const double* slot = ll_slots + 2 * ((((size_t)w * NOUT + o) * KC + k) * NS1 + j);
                 fed::dd_add(hi, lo, slot[0], slot[1]);
             }
-            out[2 * (((size_t)o * nch + k) * NV1 + j)] = hi;
-            out[2 * (((size_t)o * nch + k) * NV1 + j) + 1] = lo;
+            const int oj = (kPhi && j > G) ? j + P : j;
+            out[2 * (((size_t)o * nch + k) * NV1 + oj)] = hi;
+            out[2 * (((size_t)o * nch + k) * NV1 + oj) + 1] = lo;
         }
         if (threadIdx.x == 0) fed::stamp(comm, 6);
     } else if (warp == 0) {
@@ -665,8 +721,8 @@ extern "C" int b200_glm_tc_chunk_table(const long long* n_rows, int n_segments, 
 }
 
 // doubles in the partial array of the tensor-core kernel: one row of (hi, lo) pairs + per-warp LL slots per CTA
-extern "C" size_t b200_glm_tc_partial_row_doubles(int n_vals, int n_chains, int n_out, int n_groups) {
-    return tc::partial_row_doubles(n_vals, chains_bucket(n_chains), n_out > 0 ? n_out : 1, n_groups);
+extern "C" size_t b200_glm_tc_partial_row_doubles(int n_vals, int n_chains, int n_out, int n_groups, int n_family_params) {
+    return tc::partial_row_doubles(n_vals, chains_bucket(n_chains), n_out > 0 ? n_out : 1, n_groups, n_family_params);
 }
 
 extern "C" int b200_launch_glm_tc(const FedComm* comm, const GlmSegment* segs_dev, const GlmParams* prm, const void* tmaps,
@@ -675,12 +731,12 @@ extern "C" int b200_launch_glm_tc(const FedComm* comm, const GlmSegment* segs_de
     const int kc = chains_bucket(prm->n_chains);
     if (kc == 0) return -1;
     const CUtensorMap* maps = reinterpret_cast<const CUtensorMap*>(tmaps);
-#define LAUNCH_TC(KC)                                                                                              \
+#define LAUNCH_TC(KC, PHI)                                                                                         \
     do {                                                                                                           \
         const tc::SmemLayout L = tc::smem_layout((prm->n_features + 127) & ~127, tc::Cfg<KC>::N1, tc::Cfg<KC>::N2, comm->n_theta,  \
-                                                 prm->n_groups, KC, tc::Cfg<KC>::RB);                              \
+                                                 prm->n_groups, KC, tc::Cfg<KC>::RB, PHI ? KC * (int)sizeof(tc::PhiChain) : 0); \
         if (L.stages < 2) return -2;                                                                               \
-        cudaFuncSetAttribute(tc::fed_glm_tc_kernel<KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total); \
+        cudaFuncSetAttribute(tc::fed_glm_tc_kernel<KC, PHI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total); \
         cudaLaunchConfig_t cfg{};                                                                                  \
         cfg.gridDim = dim3(grid);                                                                                  \
         cfg.blockDim = dim3(tc::Cfg<KC>::kThreads);                                                                \
@@ -691,13 +747,20 @@ extern "C" int b200_launch_glm_tc(const FedComm* comm, const GlmSegment* segs_de
         attr[0].val.programmaticStreamSerializationAllowed = 1;                                                    \
         cfg.attrs = attr;                                                                                          \
         cfg.numAttrs = tc::use_pdl() ? 1 : 0;                                                                      \
-        cudaLaunchKernelEx(&cfg, tc::fed_glm_tc_kernel<KC>, *comm, segs_dev, *prm, maps,                           \
+        cudaLaunchKernelEx(&cfg, tc::fed_glm_tc_kernel<KC, PHI>, *comm, segs_dev, *prm, maps,                      \
                            reinterpret_cast<const GlmChunk*>(chunks_dev), n_chunks, work_counter);                 \
     } while (0)
-    if (kc == 1) LAUNCH_TC(1);
-    else if (kc == 4) LAUNCH_TC(4);
-    else if (kc == 8) LAUNCH_TC(8);
-    else LAUNCH_TC(16);
+    if (prm->n_family_params > 0) {
+        if (kc == 1) LAUNCH_TC(1, true);
+        else if (kc == 4) LAUNCH_TC(4, true);
+        else if (kc == 8) LAUNCH_TC(8, true);
+        else LAUNCH_TC(16, true);
+    } else {
+        if (kc == 1) LAUNCH_TC(1, false);
+        else if (kc == 4) LAUNCH_TC(4, false);
+        else if (kc == 8) LAUNCH_TC(8, false);
+        else LAUNCH_TC(16, false);
+    }
 #undef LAUNCH_TC
     return (int)cudaGetLastError();
 }

@@ -26,12 +26,14 @@ struct GlmParams {
     int n_segments;
     int n_features;       // P
     int ld;               // row stride of X in elements
-    int n_groups;         // G intercepts; theta = [intercept[G], beta[P]] per chain
-    int n_chains;         // K parameter vectors evaluated per launch (theta is [K][G+P])
-    int family;           // 0 = logistic (Bernoulli), 1 = Poisson (log link), 2 = Gaussian (identity, unit variance)
+    int n_groups;         // G intercepts; theta = [intercept[G], beta[P], phi[D]] per chain
+    int n_chains;         // K parameter vectors evaluated per launch (theta is [K][G+P+D])
+    int family;           // 0 = logistic (Bernoulli), 1 = Poisson (log link), 2 = Gaussian (identity, unit variance);
+                          // tensor-core kernel only: 3 = normal (sigma), 4 = Student-t (sigma, nu), 5 = negative binomial (alpha)
     long long total_tiles;
-    int n_out;            // output blocks: 1 = everything summed; > 1 = one [K][1+G+P] block per node (tensor-core kernel)
+    int n_out;            // output blocks: 1 = everything summed; > 1 = one [K][1+G+P+D] block per node (tensor-core kernel)
     int early_loads;      // tensor-core kernels: claim + load the first tiles before theta arrives (B200FED_NO_EARLY_LOADS=1: off)
+    int n_family_params;  // D fitted family parameters phi (0 for families 0-2); the result per chain is [LL, gi[G], g[P], dphi[D]]
 };
 
 // Unit of work of the dynamically scheduled tensor-core GLM kernel: n_tiles consecutive 128-row tiles of one

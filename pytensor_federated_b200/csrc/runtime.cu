@@ -44,7 +44,7 @@ int b200_launch_glm_tc(const FedComm*, const GlmSegment*, const GlmParams*, cons
                        int n_chunks, unsigned int* work_counter, int grid, cudaStream_t);
 int b200_glm_tc_prepare(const GlmSegment* segs_host, int n_segments, const GlmParams* prm, int sm_count, void** tmaps_dev,
                         void** chunks_dev, int* n_chunks);
-size_t b200_glm_tc_partial_row_doubles(int n_vals, int n_chains, int n_out, int n_groups);
+size_t b200_glm_tc_partial_row_doubles(int n_vals, int n_chains, int n_out, int n_groups, int n_family_params);
 int b200_launch_ode(const FedComm*, const OdeShard*, int, int, cudaStream_t);
 int b200_launch_glm_fp8(const FedComm*, const GlmSegment*, const GlmParams*, const void* tmaps, const void* chunks,
                         int n_chunks, unsigned int* work_counter, int grid, cudaStream_t stream);
@@ -549,9 +549,14 @@ int b200_engine_set_linreg(void* h, int n_shards, const void** x, const void** y
 
 int b200_engine_set_glm(void* h, int n_segments, const void** X, const float** y, const void** scales,
                         const long long* n_rows, const int* groups, int n_features, int ld, int n_groups,
-                        int n_chains, int family, int use_tensor_cores, const int* out_groups, int n_out) {
+                        int n_chains, int family, int use_tensor_cores, const int* out_groups, int n_out,
+                        int n_family_params) {
     Engine* e = static_cast<Engine*>(h);
     CK(cudaSetDevice(e->device));
+    if (n_family_params < 0 || (n_family_params > 0 && use_tensor_cores != 1)) {
+        g_last_error = "families with fitted parameters run on the tensor-core kernel only";
+        return -34;
+    }
     const int tile_rows = (use_tensor_cores == 1 || use_tensor_cores == 2) ? 128 : 8;
     e->glm_segs.resize(n_segments);
     long long tiles = 0;
@@ -571,9 +576,10 @@ int b200_engine_set_glm(void* h, int n_segments, const void** X, const float** y
         e->glm_segs[s] = g;
         tiles += (n_rows[s] + tile_rows - 1) / tile_rows;
     }
-    e->glm = GlmParams{n_segments, n_features, ld, n_groups, n_chains, family, tiles, n_out > 0 ? n_out : 1, early_loads_enabled() ? 1 : 0};
-    if ((long long)e->glm.n_out * n_chains * (1 + n_groups + n_features) != e->n_vals) {
-        g_last_error = "n_vals does not match n_out x n_chains x (1 + n_groups + n_features)";
+    e->glm = GlmParams{n_segments, n_features, ld, n_groups, n_chains, family, tiles, n_out > 0 ? n_out : 1,
+                       early_loads_enabled() ? 1 : 0, n_family_params};
+    if ((long long)e->glm.n_out * n_chains * (1 + n_groups + n_features + n_family_params) != e->n_vals) {
+        g_last_error = "n_vals does not match n_out x n_chains x (1 + n_groups + n_features + n_family_params)";
         return -33;
     }
     if (e->glm_segs_dev) cudaFree(e->glm_segs_dev);
@@ -605,7 +611,7 @@ int b200_engine_set_glm(void* h, int n_segments, const void** X, const float** y
             g_last_error = "tensor-core GLM path rejected this shape (rc=" + std::to_string(rc) + ")";
             return rc;
         }
-        e->tc_row_doubles = b200_glm_tc_partial_row_doubles(e->n_vals, n_chains, e->glm.n_out, n_groups);
+        e->tc_row_doubles = b200_glm_tc_partial_row_doubles(e->n_vals, n_chains, e->glm.n_out, n_groups, n_family_params);
         if (e->tc_partials) cudaFree(e->tc_partials);
         const size_t tc_doubles = (size_t)e->sm_count * e->tc_row_doubles + ((size_t)e->sm_count / 16 + 2) * e->n_vals * 2;
         CK(cudaMalloc((void**)&e->tc_partials, tc_doubles * 8));

@@ -208,5 +208,111 @@ __device__ __forceinline__ void link_loglik(int family, float y, float eta, floa
     }
 }
 
+// ------------------------------------------------------------------ families with fitted parameters phi
+// Family codes 3 = normal (sigma), 4 = student_t (sigma, nu), 5 = negative_binomial (alpha, NB2: var = mu + mu^2 / alpha).
+// They are fully normalised.  Everything that depends on phi alone is computed ONCE per chain (phi_chain, fp64):
+// fp32 helpers for the per-row maths, and the per-row constants c of the log-likelihood and of d/dphi, which the
+// kernel adds in fp64 as (valid rows of a chunk) x c instead of summing them row by row.
+struct PhiChain {
+    double c_ll, c_d0, c_d1;   // per-row constants of LL, dLL/dphi0, dLL/dphi1
+    float p[4];                // fp32 helpers of the per-row maths (family-specific, see phi_chain)
+};
+
+// Digamma for x > 0: recurrence up to x >= 10, then the asymptotic series (error < 1e-13 there).
+template <typename T>
+__host__ __device__ inline T digamma(T x) {
+    T acc = 0;
+    while (x < T(10)) {
+        acc -= T(1) / x;
+        x += T(1);
+    }
+    const T inv = T(1) / x, inv2 = inv * inv;
+    const T series = inv2 * (T(1) / 12 - inv2 * (T(1) / 120 - inv2 * (T(1) / 252 - inv2 * (T(1) / 240 - inv2 * (T(1) / 132)))));
+    return acc + log(x) - T(0.5) * inv - series;
+}
+
+__device__ inline PhiChain phi_chain(int family, const float* phi) {
+    PhiChain c{0.0, 0.0, 0.0, {0.f, 0.f, 0.f, 0.f}};
+    const double s = phi[0];
+    if (family == 3) {
+        c.p[0] = (float)(1.0 / s);
+        c.c_ll = -log(s) - 0.918938533204672742;
+        c.c_d0 = -1.0 / s;
+    } else if (family == 4) {
+        const double nu = phi[1];
+        c.p[0] = (float)(1.0 / s);
+        c.p[1] = phi[1];
+        c.p[2] = (float)(1.0 / nu);
+        c.p[3] = (float)(nu + 1.0);
+        c.c_ll = lgamma(0.5 * (nu + 1.0)) - lgamma(0.5 * nu) - 0.5 * log(nu * 3.14159265358979323846) - log(s);
+        c.c_d0 = -1.0 / s;
+        c.c_d1 = 0.5 * (digamma(0.5 * (nu + 1.0)) - digamma(0.5 * nu) - 1.0 / nu);
+    } else if (family == 5) {
+        c.p[0] = phi[0];
+        c.p[1] = (float)(1.0 / s);
+        c.p[2] = (float)log(s);
+    }
+    return c;
+}
+
+// Counts below this use the exact short sums  lgamma(y+a) - lgamma(a) - lgamma(y+1) = sum_{j<y} log((a+j)/(j+1))  and
+// psi(y+a) - psi(a) = sum_{j<y} 1/(a+j)  in fp32; larger counts take lgamma / digamma in fp64 (the fp32 difference of
+// two lgammas near 1e3..1e4 cancels catastrophically: lgammaf(1000) ~ 5905 has an ulp of ~5e-4).
+constexpr int kNbShortSum = 16;
+
+__device__ __forceinline__ void nb_count_terms(float y, float a, float& lg, float& dg) {
+    const int n = (int)y;
+    if (n < kNbShortSum) {
+        float lsum = 0.f, dsum = 0.f, prod = 1.f;
+        for (int j = 0; j < n; ++j) {
+            const float aj = a + (float)j;
+            prod *= __fdividef(aj, (float)(j + 1));
+            dsum += __fdividef(1.f, aj);
+            if (j & 1) {   // pairs of ratios: no fp32 overflow for a up to ~1e19
+                lsum += __logf(prod);
+                prod = 1.f;
+            }
+        }
+        lg = lsum + __logf(prod);
+        dg = dsum;
+    } else {
+        const double yd = y, ad = a;
+        lg = (float)(lgamma(yd + ad) - lgamma(ad) - lgamma(yd + 1.0));
+        dg = (float)(digamma(yd + ad) - digamma(ad));
+    }
+}
+
+// Per row: the phi-free part of LL, r = dLL/deta and the row parts of dLL/dphi (the per-chain constants of
+// PhiChain are added per chunk).  p = PhiChain::p of the chain.
+__device__ __forceinline__ void link_loglik_phi(int family, float y, float eta, const float* p, float& ll, float& r,
+                                                float& d0, float& d1) {
+    if (family == 3) {                               // p = (1/sigma)
+        const float z = (y - eta) * p[0];
+        ll = -0.5f * z * z;
+        r = z * p[0];
+        d0 = z * z * p[0];
+        d1 = 0.f;
+    } else if (family == 4) {                        // p = (1/sigma, nu, 1/nu, nu + 1)
+        const float z = (y - eta) * p[0];
+        const float z2 = z * z;
+        const float l1p = log1pf(z2 * p[2]);
+        const float w = __fdividef(p[3], p[1] + z2);  // (nu + 1) / (nu + z^2)
+        ll = -0.5f * p[3] * l1p;
+        r = w * z * p[0];
+        d0 = w * z2 * p[0];
+        d1 = 0.5f * (w * z2 * p[2] - l1p);
+    } else {                                         // p = (alpha, 1/alpha, log alpha)
+        const float mu = expf(eta);
+        const float l1 = log1pf(mu * p[1]);          // log((alpha + mu) / alpha)
+        const float inv = __fdividef(1.f, p[0] + mu);
+        float lg, dg;
+        nb_count_terms(y, p[0], lg, dg);
+        ll = lg - p[0] * l1 + y * (eta - p[2] - l1);
+        r = p[0] * (y - mu) * inv;
+        d0 = dg - l1 + (mu - y) * inv;
+        d1 = 0.f;
+    }
+}
+
 
 }  // namespace tc

@@ -35,7 +35,8 @@ class NodeFederation:
     * ``OdeShards(..., node_ids=, n_nodes=)`` — node = the shards with that node id; input ``(theta,)``; every
       node may be given its own parameter vector.
     * ``GlmShards(..., node_ids=, n_nodes=)`` — node = the segments with that node id; inputs
-      ``(intercepts[G], beta[P])``.  Nodes that are given the same parameters (the usual federated GLM)
+      ``(intercepts[G], beta[P])`` — plus ``phi[D]`` for the families with fitted parameters (negative binomial,
+      Student-t, normal).  Nodes that are given the same parameters (the usual federated GLM)
       share a chain; *distinct* parameter vectors occupy one chain each, so the model must have been built
       with ``n_chains >=`` the number of distinct vectors of a call.
 
@@ -95,14 +96,22 @@ class NodeFederation:
 
     def _evaluate_glm(self, requests):
         m = self.engine.model
-        G, K = m.n_groups, m.n_chains
-        chains: Dict[bytes, int] = {}      # distinct parameter vector -> chain
+        G, K, D = m.n_groups, m.n_chains, m.n_family_params
+        GP = G + m.n_features
+        chains: Dict[bytes, int] = {}      # distinct parameter vector [intercept, beta, phi] -> chain
         rows: List[np.ndarray] = []
         chain_of: Dict[int, int] = {}
         shapes: Dict[int, tuple] = {}
-        for node, (intercept, beta) in requests.items():
-            ic = np.asarray(intercept, dtype=np.float32)
-            vec = np.concatenate([ic.reshape(G), np.asarray(beta, dtype=np.float32).reshape(m.n_features)])
+        phi_shapes: Dict[int, tuple] = {}
+        for node, inputs in requests.items():
+            if len(inputs) != m.n_inputs:
+                raise ValueError(f"node {node}: the {m.family} GLM takes {m.n_inputs} inputs, got {len(inputs)}")
+            ic = np.asarray(inputs[0], dtype=np.float32)
+            parts = [ic.reshape(G), np.asarray(inputs[1], dtype=np.float32).reshape(m.n_features)]
+            if D:
+                parts.append(np.asarray(inputs[2], dtype=np.float32).reshape(D))
+                phi_shapes[node] = np.shape(inputs[2])   # a scalar phi (D = 1) gets a scalar gradient
+            vec = np.concatenate(parts)
             key = vec.tobytes()
             if key not in chains:
                 if len(rows) == K:
@@ -115,12 +124,14 @@ class NodeFederation:
             chain_of[node] = chains[key]
             shapes[node] = ic.shape
         theta = np.stack(rows + [rows[0]] * (K - len(rows)))                       # unused chains repeat the first
-        inputs = [theta[:, :G], theta[:, G:]] if K > 1 else [theta[0, :G], theta[0, G:]]
-        per = m.per_node(self.engine.evaluate_raw(inputs))                         # [n_nodes, K, 1 + G + P]
+        th = theta if K > 1 else theta[0]
+        inputs = [th[..., :G], th[..., G:GP]] + ([th[..., GP:]] if D else [])
+        per = m.per_node(self.engine.evaluate_raw(inputs))                         # [n_nodes, K, 1 + G + P + D]
         out = {}
         for node in requests:
             v = per[node, chain_of[node]]
-            out[node] = (np.array(v[0]), [v[1 : 1 + G].reshape(shapes[node]).copy(), v[1 + G :].copy()])
+            grads = [v[1 : 1 + G].reshape(shapes[node]).copy(), v[1 + G : 1 + GP].copy()]
+            out[node] = (np.array(v[0]), grads + ([v[1 + GP :].reshape(phi_shapes[node]).copy()] if D else []))
         return out
 
     def evaluate_node(self, node: int, *inputs) -> Tuple[np.ndarray, List[np.ndarray]]:
@@ -146,7 +157,8 @@ class NodeFederation:
         * linear regression: ``f(intercepts, slopes) -> (logp, [d_intercepts, d_slopes])``, each argument a vector
           ``[n_nodes]`` or a scalar shared by all nodes (its gradient is then the sum over the nodes);
         * ODE: ``f(theta[n_nodes, n_params]) -> (logp, [d_theta])``;
-        * GLM (parameters shared by the nodes): ``f(intercept, beta) -> (logp, [d_intercept, d_beta])``.
+        * GLM (parameters shared by the nodes): ``f(intercept, beta) -> (logp, [d_intercept, d_beta])``, and for the
+          families with fitted parameters ``f(intercept, beta, phi) -> (logp, [d_intercept, d_beta, d_phi])``.
 
         With :meth:`all_nodes_op` the model graph has ONE federated node instead of one per data holder, so the
         Python cost of a model evaluation no longer grows with the size of the federation."""
@@ -166,6 +178,12 @@ class NodeFederation:
                     th = np.broadcast_to(np.asarray(theta, dtype=np.float64), (self.n_nodes, m.n_params))
                     per = m.per_node(eng.evaluate_raw([th]))
                     return np.asarray(per[:, 0].sum()), [per[:, 1:].copy()]
+        elif eng.model.n_family_params:
+            def func(intercept, beta, phi):
+                with self._lock:
+                    self.n_launches += 1
+                    logp, *grads = eng.evaluate(intercept, beta, phi)
+                    return logp, grads
         else:
             def func(intercept, beta):
                 with self._lock:

@@ -6,6 +6,9 @@ bf16 design matrix* and *hierarchical GLM, 8 partial-pooling groups, fp8 block-s
 matrix*.  ``theta = [intercept[G], beta[P]]`` (float32) per chain; a segment (shard) uses
 ``intercept[group]``, so G = 1 is the pooled GLM and G = #shards the partial-pooling one.
 Result per chain: ``[LL, dLL/dintercept[G], dLL/dbeta[P]]`` (float64).
+
+The families with fitted parameters (``normal``, ``student_t``, ``negative_binomial``) append their D
+parameters phi: ``theta = [intercept[G], beta[P], phi[D]]`` and ``[LL, d intercept[G], d beta[P], d phi[D]]``.
 """
 from __future__ import annotations
 
@@ -16,7 +19,16 @@ import numpy as np
 
 from .base import ShardModel
 
-FAMILIES = {"logistic": 0, "poisson": 1, "gaussian": 2}
+FAMILIES = {"logistic": 0, "poisson": 1, "gaussian": 2, "normal": 3, "student_t": 4, "negative_binomial": 5}
+
+#: Families whose parameters phi are inferred along with the coefficients (tensor-core kernel only).  They are
+#: fully normalised: the log-likelihood equals the scipy log density summed over the rows —
+#: ``norm.logpdf(y, eta, sigma)``, ``t.logpdf(y, nu, eta, sigma)`` and, with ``mu = exp(eta)``,
+#: ``nbinom.logpmf(y, alpha, alpha / (alpha + mu))`` (NB2, ``var = mu + mu^2 / alpha``, PyMC's
+#: ``NegativeBinomial(mu, alpha)``).  ``gaussian`` keeps its unit variance.
+FAMILY_PARAMS = {"normal": ("sigma",), "student_t": ("sigma", "nu"), "negative_binomial": ("alpha",)}
+
+_TC_SHAPES = "bf16 design matrix, P % 8 == 0, 8 <= P <= 384, K <= 16 chains, 16-byte aligned rows"
 
 
 def _family_code(family) -> int:
@@ -37,6 +49,11 @@ class GlmShards(ShardModel):
         Total number of intercepts G in the federation.
     n_chains
         Parameter vectors evaluated per call (K).  ``K > 1`` needs the tensor-core kernel.
+    family
+        ``"logistic"``, ``"poisson"``, ``"gaussian"`` (unit variance), or one of the families with fitted
+        parameters (:data:`FAMILY_PARAMS`): ``"normal"`` (sigma), ``"student_t"`` (sigma, nu) and
+        ``"negative_binomial"`` (alpha).  These take a third input ``phi`` and return ``d_phi``; they run on the
+        tensor-core kernel only.  A :class:`~pytensor_federated_b200.models.custom.CustomFamily` is accepted too.
     kernel
         ``"simt"`` (one chain, any P % 8 == 0 up to 512), ``"tc"`` (tcgen05 + TMA: bf16, any P % 8 == 0 up to
         384 — the tile is padded to whole 128-feature blocks by TMA's zero fill —, up to 16 chains) or ``"auto"``.
@@ -82,8 +99,15 @@ class GlmShards(ShardModel):
             if X.dim() != 2 or X.shape[1] != self.n_features or X.stride(1) != 1 or X.stride(0) != self.ld:
                 raise ValueError("all design matrices must be row-major [n, P] with one row stride")
         self.device = X0.device
-        self.n_inputs = 2
-        self.n_params = self.n_groups + self.n_features
+        #: names of the fitted family parameters phi, e.g. ``("sigma", "nu")`` (empty for the other families)
+        self.family_param_names = FAMILY_PARAMS.get(family, ()) if isinstance(family, str) else ()
+        self.n_family_params = len(self.family_param_names)
+        if family == "negative_binomial":
+            for y in self.ys:
+                if y.numel() and not bool(((y >= 0) & (y == torch.floor(y))).all()):
+                    raise ValueError("negative_binomial needs non-negative integer counts y")
+        self.n_inputs = 3 if self.n_family_params else 2
+        self.n_params = self.n_groups + self.n_features + self.n_family_params
         self.n_theta_words = self.n_chains * self.n_params
         if (node_ids is None) != (n_nodes is None):
             raise ValueError("node_ids and n_nodes come together")
@@ -100,26 +124,44 @@ class GlmShards(ShardModel):
     # -- packing ---------------------------------------------------------------------------
     def call_context(self, inputs):
         """``(batched, intercept shape)`` of one call: a 2-D ``beta`` means one row per chain."""
-        intercept, beta = inputs
+        intercept, beta = inputs[0], inputs[1]
         return (np.ndim(beta) == 2, np.shape(intercept))
+
+    def _split_inputs(self, inputs):
+        """``(intercept, beta, phi or None)``, checking the number of inputs against the family."""
+        if len(inputs) != self.n_inputs:
+            want = "(intercept, beta, phi)" if self.n_family_params else "(intercept, beta)"
+            raise ValueError(f"the {self.family!s} GLM takes {self.n_inputs} inputs {want}, got {len(inputs)}")
+        return inputs[0], inputs[1], (inputs[2] if self.n_family_params else None)
+
+    def _check_phi(self, phi) -> np.ndarray:
+        ph = np.asarray(phi, dtype=np.float64).reshape(self.n_chains, self.n_family_params)
+        if not np.all(np.isfinite(ph) & (ph > 0)):
+            raise ValueError(f"family parameters {self.family_param_names} must be finite and > 0, got {ph.tolist()}")
+        return ph
 
     _pack_views = None
 
     def pack_theta(self, inputs, out: np.ndarray):
-        intercept, beta = inputs
+        intercept, beta, phi = self._split_inputs(inputs)
         views = self._pack_views
         if views is None or views[0] is not out:
             # float32 windows into the staging buffer, built once per buffer (this runs on every evaluation)
             th = out.view(np.float32).reshape(self.n_chains, self.n_params)
-            views = self._pack_views = (out, th[:, : self.n_groups], th[:, self.n_groups :])
+            G, GP = self.n_groups, self.n_groups + self.n_features
+            views = self._pack_views = (out, th[:, :G], th[:, G:GP], th[:, GP:])
         ic = intercept if type(intercept) is np.ndarray else np.asarray(intercept)
         bt = beta if type(beta) is np.ndarray else np.asarray(beta)
         batched = bt.ndim == 2
         ctx = (batched, ic.shape)
+        if phi is not None:
+            ph = self._check_phi(phi)   # before anything is written: a rejected call leaves the buffer alone
         self._batched, self._icpt_shape = ctx
         # the assignments convert to float32 while they copy
         views[1][...] = ic.reshape(self.n_chains, -1) if batched else ic.reshape(1, -1)
         views[2][...] = bt.reshape(self.n_chains, self.n_features)
+        if phi is not None:
+            views[3][...] = ph
         return ctx
 
     _batched = False
@@ -133,17 +175,19 @@ class GlmShards(ShardModel):
         return ctx
 
     def per_node(self, vals: np.ndarray) -> np.ndarray:
-        """The reduced vector as ``[n_nodes, n_chains, 1 + G + P]`` (``[LL, d intercepts, d beta]`` per block)."""
+        """The reduced vector as ``[n_nodes, n_chains, 1 + G + P + D]`` (``[LL, d intercepts, d beta, d phi]`` per block)."""
         return np.asarray(vals, dtype=np.float64).reshape(self.n_nodes, self.n_chains, 1 + self.n_params)
 
     def unpack_result(self, vals: np.ndarray, ctx=None) -> List[np.ndarray]:
         v = self.per_node(vals).sum(axis=0) if self.n_nodes > 1 else np.asarray(vals, dtype=np.float64).reshape(self.n_chains, 1 + self.n_params)
-        G = self.n_groups
+        G, GP = self.n_groups, self.n_groups + self.n_features
         batched, icpt_shape = ctx if ctx is not None else (self._batched, self._icpt_shape)
         if batched:
-            return [v[:, 0].copy(), v[:, 1 : 1 + G].reshape((self.n_chains,) + tuple(icpt_shape[1:])).copy(),
-                    v[:, 1 + G :].copy()]
-        return [np.asarray(v[0, 0]), v[0, 1 : 1 + G].reshape(icpt_shape).copy(), v[0, 1 + G :].copy()]
+            out = [v[:, 0].copy(), v[:, 1 : 1 + G].reshape((self.n_chains,) + tuple(icpt_shape[1:])).copy(),
+                   v[:, 1 + G : 1 + GP].copy()]
+            return out + [v[:, 1 + GP :].copy()] if self.n_family_params else out
+        out = [np.asarray(v[0, 0]), v[0, 1 : 1 + G].reshape(icpt_shape).copy(), v[0, 1 + G : 1 + GP].copy()]
+        return out + [v[0, 1 + GP :].copy()] if self.n_family_params else out
 
     # -- native ----------------------------------------------------------------------------
     def use_tensor_cores(self):
@@ -152,6 +196,14 @@ class GlmShards(ShardModel):
         import torch
 
         X0 = self.Xs[0]
+        tc_ok = (X0.dtype == torch.bfloat16 and self.n_features % 8 == 0 and 8 <= self.n_features <= 384
+                 and self.n_chains <= 16 and all(X.data_ptr() % 16 == 0 for X in self.Xs) and self.ld % 8 == 0)
+        if self.n_family_params:
+            # the families with fitted parameters exist on the tensor-core kernel only
+            if self.kernel not in ("tc", "auto") or not tc_ok:
+                raise ValueError(f"the {self.family} family runs on the tensor-core kernel only ({_TC_SHAPES}); "
+                                 f"kernel={self.kernel!r}, dtype {X0.dtype}, P = {self.n_features}, K = {self.n_chains}")
+            return 1
         if hasattr(self.family, "code_id"):  # user-compiled likelihood: general-shape kernel
             if X0.dtype not in (torch.bfloat16, torch.float32) or self.n_chains != 1 or self.n_features > 1024:
                 raise ValueError("custom likelihoods need a bf16/fp32 design matrix, one chain and P <= 1024")
@@ -170,8 +222,6 @@ class GlmShards(ShardModel):
         # auto: the tcgen05 kernel wherever its shape constraints hold (it is faster even for one chain:
         # TMA streaming + the X tile reused from smem for both GEMMs), then SIMT, then the general kernel
         bf16 = X0.dtype == torch.bfloat16
-        tc_ok = (bf16 and self.n_features % 8 == 0 and 8 <= self.n_features <= 384 and self.n_chains <= 16
-                 and all(X.data_ptr() % 16 == 0 for X in self.Xs) and self.ld % 8 == 0)
         if tc_ok:
             return 1
         if self.n_chains > 1:
@@ -209,7 +259,7 @@ class GlmShards(ShardModel):
         native.check(
             lib.b200_engine_set_glm(
                 handle, n, Xp, yp, sp, rows, grp, self.n_features, self.ld, self.n_groups,
-                self.n_chains, _family_code(self.family), code, out_grp, self.n_nodes,
+                self.n_chains, _family_code(self.family), code, out_grp, self.n_nodes, self.n_family_params,
             ),
             "set_glm",
         )
@@ -224,12 +274,14 @@ class GlmShards(ShardModel):
         import torch
 
         dtype = dtype or torch.float32
-        intercept, beta = inputs
+        intercept, beta, phi = self._split_inputs(inputs)
         self._note_shapes(inputs)
         ic = torch.as_tensor(np.asarray(intercept, dtype=np.float64)).reshape(self.n_chains, -1)
         bt = torch.as_tensor(np.asarray(beta, dtype=np.float64)).reshape(self.n_chains, self.n_features)
         full = torch.zeros(self.n_nodes, self.n_chains, 1 + self.n_params, dtype=torch.float64, device=self.device)
         B = bt.to(self.device, dtype)                              # [K, P]
+        ph = torch.as_tensor(self._check_phi(phi)).to(self.device, dtype) if phi is not None else None   # [K, D]
+        GP = self.n_groups + self.n_features
         for si, (X, y, g) in enumerate(zip(self.Xs, self.ys, self.groups)):
             out = full[self.node_ids[si] if self.node_ids is not None else 0]
             icg = ic[:, g].to(self.device, dtype)
@@ -242,6 +294,10 @@ class GlmShards(ShardModel):
                     if self.family.torch_fn is None:
                         raise ValueError("this CustomFamily has no torch_fn oracle")
                     ll, r = self.family.torch_fn(yy, eta)
+                elif ph is not None:
+                    ll, r, dphi = _phi_family_terms(self.family, yy, eta, ph)
+                    for j, dj in enumerate(dphi):
+                        out[:, 1 + GP + j] += dj.double().sum(0)
                 elif self.family == "logistic":
                     ll = yy * eta - torch.nn.functional.softplus(eta)
                     r = yy - torch.sigmoid(eta)
@@ -255,7 +311,7 @@ class GlmShards(ShardModel):
                     r = d
                 out[:, 0] += ll.double().sum(0)
                 out[:, 1 + g] += r.double().sum(0)
-                out[:, 1 + self.n_groups :] += (r.T @ Xf).double()
+                out[:, 1 + self.n_groups : 1 + GP] += (r.T @ Xf).double()
         return full.reshape(-1).cpu().numpy()
 
     def _dequant_rows(self, seg: int, r0: int, r1: int):
@@ -271,7 +327,7 @@ class GlmShards(ShardModel):
         design matrix twice; no custom kernels."""
         import torch
 
-        if self.Xs[0].dtype != torch.bfloat16:
+        if self.Xs[0].dtype != torch.bfloat16 or self.n_family_params:
             return self.reference_partial(inputs)
         intercept, beta = inputs
         self._note_shapes(inputs)
@@ -302,6 +358,36 @@ class GlmShards(ShardModel):
 
     def flops_per_eval(self) -> int:
         return int(4 * self.n_rows * self.n_features * self.n_chains)
+
+
+def _phi_family_terms(family: str, y, eta, phi):
+    """Per-row ``(ll, dll/deta, [dll/dphi_j])`` of a family with fitted parameters (``phi`` ``[K, D]``)."""
+    import math
+
+    import torch
+
+    if family == "normal":
+        s = phi[:, 0]
+        z = (y - eta) / s
+        return -0.5 * z * z - torch.log(s) - 0.5 * math.log(2 * math.pi), z / s, [(z * z - 1) / s]
+    if family == "student_t":
+        s, nu = phi[:, 0], phi[:, 1]
+        d = y - eta
+        z2 = (d / s) ** 2
+        l1p = torch.log1p(z2 / nu)
+        ll = (torch.lgamma((nu + 1) / 2) - torch.lgamma(nu / 2) - 0.5 * torch.log(nu * math.pi) - torch.log(s)
+              - (nu + 1) / 2 * l1p)
+        r = (nu + 1) * d / (nu * s * s + d * d)
+        d_s = ((nu + 1) * z2 / (nu + z2) - 1) / s
+        d_nu = 0.5 * (torch.digamma((nu + 1) / 2) - torch.digamma(nu / 2) - 1 / nu - l1p + (nu + 1) * z2 / (nu * (nu + z2)))
+        return ll, r, [d_s, d_nu]
+    a = phi[:, 0]                                        # negative_binomial
+    mu = torch.exp(eta)
+    l1 = torch.log1p(mu / a)
+    ll = torch.lgamma(y + a) - torch.lgamma(a) - torch.lgamma(y + 1) - a * l1 + y * (eta - torch.log(a + mu))
+    r = a * (y - mu) / (a + mu)
+    d_a = torch.digamma(y + a) - torch.digamma(a) - l1 + (mu - y) / (a + mu)
+    return ll, r, [d_a]
 
 
 def quantize_block_fp8(X, block: int = 32):
@@ -376,6 +462,9 @@ class Fp8GlmShards(GlmShards):
                  family: str = "logistic", node_ids=None, n_nodes=None) -> None:
         if not 1 <= n_chains <= 3:
             raise ValueError("the fp8 kernel batches at most 3 chains per launch")
+        if family in FAMILY_PARAMS:
+            raise ValueError(f"the fp8 kernel has no {family} family: families with fitted parameters run on the "
+                             f"bf16 tensor-core kernel ({_TC_SHAPES})")
         super().__init__(Xqs, ys, groups=groups, n_groups=n_groups, family=family, n_chains=n_chains, kernel="fp8",
                          scales=scales, node_ids=node_ids, n_nodes=n_nodes)
         self._kernel_scales = [pack_tile_scales(s, self.n_features) for s in self.scales]
@@ -441,3 +530,48 @@ def synth_logistic_shard_fp8(n_rows: int, n_features: int, *, seed: int, device,
         p = torch.sigmoid(xd @ (beta_true / col_scale) + 0.3)
         y[r0:r1] = (torch.rand(r1 - r0, generator=gen, device=device) < p).float()
     return Xq, scales, y
+
+
+def synth_glm_shard(n_rows: int, n_features: int, *, family: str = "logistic", phi=(), seed: int, device,
+                    chunk_rows: int = 1 << 20, beta_scale: float = 0.05, intercept: float = 0.3, beta_true=None):
+    """Synthetic shard of any built-in family, generated on the device in chunks: bf16 ``X ~ N(0,1)``,
+    ``eta = X beta* + intercept`` and ``y`` drawn from the family with parameters ``phi`` (``(sigma,)``,
+    ``(sigma, nu)`` or ``(alpha,)``; the negative binomial as a gamma-Poisson mixture).  ``beta*`` is drawn
+    (``N(0, beta_scale^2)``) unless ``beta_true`` is given — nodes of one federation share it.  Returns
+    ``(X, y, beta_true)``.  Draws come from a seeded fork of torch's generator, so the global state is untouched."""
+    import torch
+
+    names = FAMILY_PARAMS.get(family, ())
+    phi = tuple(float(v) for v in np.atleast_1d(np.asarray(phi, dtype=np.float64)))
+    if family not in FAMILIES or len(phi) != len(names):
+        raise ValueError(f"family {family!r} takes parameters {names}, got {phi}")
+    device = torch.device(device)
+    with torch.random.fork_rng(devices=[device] if device.type == "cuda" else []):
+        torch.manual_seed(seed)
+        drawn = torch.randn(n_features, device=device) * beta_scale
+        beta_true = (drawn if beta_true is None else torch.as_tensor(beta_true, device=device)).float()
+        X = torch.empty(n_rows, n_features, dtype=torch.bfloat16, device=device)
+        y = torch.empty(n_rows, dtype=torch.float32, device=device)
+        for r0 in range(0, n_rows, chunk_rows):
+            r1 = min(n_rows, r0 + chunk_rows)
+            xb = torch.randn(r1 - r0, n_features, device=device, dtype=torch.float32).to(torch.bfloat16)
+            X[r0:r1] = xb
+            eta = xb.float() @ beta_true + intercept
+            n = r1 - r0
+            if family == "logistic":
+                yb = (torch.rand(n, device=device) < torch.sigmoid(eta)).float()
+            elif family == "poisson":
+                yb = torch.poisson(torch.exp(eta))
+            elif family == "gaussian":
+                yb = eta + torch.randn(n, device=device)
+            elif family == "normal":
+                yb = eta + phi[0] * torch.randn(n, device=device)
+            elif family == "student_t":
+                chi2 = 2.0 * torch._standard_gamma(torch.full((n,), phi[1] / 2, device=device))
+                yb = eta + phi[0] * torch.randn(n, device=device) / torch.sqrt(chi2 / phi[1])
+            else:                                                  # negative_binomial
+                alpha = phi[0]
+                rate = torch._standard_gamma(torch.full((n,), alpha, device=device)) * (torch.exp(eta) / alpha)
+                yb = torch.poisson(rate)
+            y[r0:r1] = yb.float()
+    return X, y, beta_true

@@ -65,7 +65,7 @@ def _declare(lib: C.CDLL) -> None:
     )
     sig(
         "b200_engine_set_glm", C.c_int, C.c_void_p, C.c_int, c_void_pp, c_void_pp, c_void_pp, c_ll_p,
-        c_int_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, c_int_p, C.c_int,
+        c_int_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, c_int_p, C.c_int, C.c_int,
     )
     sig(
         "b200_engine_set_ode", C.c_int, C.c_void_p, C.c_int, c_void_pp, c_void_pp, c_void_pp, c_int_p,

@@ -518,9 +518,10 @@ def default_inputs_from_words(model: ShardModel, words: np.ndarray):
         return th[:, 0].copy(), th[:, 1].copy()
     if isinstance(model, GlmShards):
         th = words.view(np.float32).reshape(model.n_chains, model.n_params)
-        if model.n_chains == 1:
-            return th[0, : model.n_groups].copy(), th[0, model.n_groups :].copy()
-        return th[:, : model.n_groups].copy(), th[:, model.n_groups :].copy()
+        G, GP = model.n_groups, model.n_groups + model.n_features
+        rows = th[0] if model.n_chains == 1 else th
+        inputs = (rows[..., :G].copy(), rows[..., G:GP].copy())
+        return inputs + (rows[..., GP:].copy(),) if model.n_family_params else inputs
     if isinstance(model, OdeShards):
         return model.inputs_from_words(words)
     raise FederationError(f"{type(model).__name__} must implement inputs_from_words()")

@@ -158,32 +158,46 @@ def glm_batch_fn(engine, n_groups: int) -> BatchFn:
     """Adapts a multi-chain ``FederatedEngine(GlmShards(..., n_chains=K))`` to the batched signature
     with ``theta = [intercept[G], beta[P]]`` per chain (flat prior; add priors by wrapping).
 
+    For the families with fitted parameters phi (``normal``, ``student_t``, ``negative_binomial``) the sampler
+    works on the unconstrained ``theta = [intercept[G], beta[P], log phi[D]]``: phi = exp(theta[G+P:]), the
+    gradient is taken through the chain rule and the log-Jacobian ``sum(log phi)`` is added to logp, so a flat
+    prior on log phi is the improper prior ``1 / phi`` on phi.
+
     Any number of chains may be passed: the kernel's capacity per launch is ``K`` (at most 16 for the bf16
     tensor-core kernel, 3 for the fp8 kernel); more chains are evaluated in ``ceil(chains / K)`` launches and a
     short last tile is padded by repeating its last chain, so 64 chains on a K = 16 engine cost four passes over the
     data instead of sixty-four."""
     cap = int(getattr(engine.model, "n_chains", 1))
+    D = int(getattr(engine.model, "n_family_params", 0))
 
-    def tile(theta: np.ndarray):
-        logp, d_ic, d_beta = engine.evaluate(theta[:, :n_groups], theta[:, n_groups:])
-        return np.asarray(logp).reshape(-1), np.concatenate([np.asarray(d_ic).reshape(cap, -1), np.asarray(d_beta).reshape(cap, -1)], axis=1)
+    def evaluate(theta: np.ndarray):
+        """theta ``[cap, G+P(+D)]`` -> (logp ``[cap]``, grad ``[cap, G+P(+D)]``) in the sampler's coordinates."""
+        single = cap == 1   # single-chain engines take unbatched inputs
+        rows = theta[0] if single else theta
+        G = n_groups
+        if not D:
+            logp, d_ic, d_beta = engine.evaluate(rows[..., :G], rows[..., G:])
+            return np.asarray(logp).reshape(-1), np.concatenate(
+                [np.asarray(d_ic).reshape(cap, -1), np.asarray(d_beta).reshape(cap, -1)], axis=1)
+        log_phi = rows[..., -D:]
+        phi = np.exp(log_phi)
+        logp, d_ic, d_beta, d_phi = engine.evaluate(rows[..., :G], rows[..., G:-D], phi)
+        logp = np.asarray(logp).reshape(-1) + np.asarray(log_phi).reshape(cap, D).sum(axis=1)
+        d_log_phi = np.asarray(d_phi).reshape(cap, D) * phi.reshape(cap, D) + 1.0
+        return logp, np.concatenate([np.asarray(d_ic).reshape(cap, -1), np.asarray(d_beta).reshape(cap, -1), d_log_phi], axis=1)
 
     def fn(theta: np.ndarray):
         theta = np.asarray(theta)
         n = theta.shape[0]
         if n == cap and cap > 1:
-            return tile(theta)
+            return evaluate(theta)
         logps, grads = [], []
         for first in range(0, n, cap):
             block = theta[first : first + cap]
             k = block.shape[0]
             if k < cap:
                 block = np.concatenate([block, np.repeat(block[-1:], cap - k, axis=0)], axis=0)
-            if cap == 1:   # single-chain engines take unbatched inputs
-                logp, d_ic, d_beta = engine.evaluate(block[0, :n_groups], block[0, n_groups:])
-                lp, gr = np.asarray(logp).reshape(1), np.concatenate([np.asarray(d_ic).reshape(-1), np.asarray(d_beta)])[None]
-            else:
-                lp, gr = tile(block)
+            lp, gr = evaluate(block)
             logps.append(lp[:k])
             grads.append(gr[:k])
         return np.concatenate(logps), np.concatenate(grads, axis=0)
